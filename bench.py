@@ -3,6 +3,7 @@
 Mixtral-8x7B geometry (32 layers, bf16, random-init weights, synthetic inputs).
 
     python bench.py --gpus 1 --steps K --warmup W              # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                     # + the last timed step's outputs as DIR/<name>.npy
     python bench.py --impl reference --gpus 1 --steps K ...    # the reference algorithm on the host CPU (oracle port)
     torchrun --nproc-per-node N bench.py --gpus N ...          # N independent replicas (request parallel, weak scaling)
 
@@ -20,6 +21,7 @@ import threading
 import time
 from pathlib import Path
 
+import numpy as np
 import torch
 
 ROOT = Path(__file__).resolve().parent
@@ -250,6 +252,16 @@ def workload_config(cfg, args, n):
             "l2_policy": "inputs larger than L2 (93.7 GB of weights streamed every step)"}
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as <out_dir>/<name>.npy (float32, or float64 as given), so that two builds run with the same
+    arguments, and hence the same seeded weights and inputs, can be compared output for output."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        assert t.dtype in (torch.float32, torch.float64), name
+        np.save(d / f"{name}.npy", t.detach().cpu().numpy())
+
+
 # ================================================================================================ expert-parallel record
 def ep_inputs(cfg, S_target=4096, n_frames=8):
     """BASELINE configs[3]: 8 video frames (448 x 448) + 10 s audio + text filling the sequence to S = 4096."""
@@ -398,6 +410,7 @@ def run_b200(args):
         torch.cuda.synchronize()
 
     ev = lambda: torch.cuda.Event(enable_timing=True)
+    last = {}           # the latest step's prefill output, kept by reference for --dump-outputs
 
     def device_step():
         e = [ev() for _ in range(4)]
@@ -405,7 +418,9 @@ def run_b200(args):
         emb, lens = model._embeds_for(ids, images_d, {"audios": feats_d, "lengths": lengths})
         e[1].record()
         llm.reset()
-        llm.prefill(emb[0, : lens[0]].contiguous(), slot=0)
+        x = emb[0, : lens[0]].contiguous()
+        llm.prefill(x, slot=0)          # x is the residual stream: it ends as the last layer's hidden states
+        last["prefill_hidden"] = x
         e[2].record()
         for _ in range(NT):
             llm.decode_step(1, use_graph=True)
@@ -452,6 +467,12 @@ def run_b200(args):
     launches = eager_launches + args.steps * NT * llm.launches_per_decode_step + enc_replayed
     toks = llm.generated_tokens(0)
     assert len(toks) == NT and all(0 <= t < cfg.llm.vocab_size for t in toks)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {
+            "generated_ids": torch.tensor(toks, dtype=torch.float64),
+            "prefill_hidden": last["prefill_hidden"].float(),          # [S, H]: every prompt position, last layer
+            "decode_hidden": llm.d_h[0].float(),                       # [H]: last decode step, last layer
+        })
 
     # ---- e2e: the public generate() with HOST inputs (pinned), H2D + D2H inside the timed region ------------
     barrier()
@@ -655,6 +676,10 @@ def main():
     ap.add_argument("--no-long-prefill", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the full-depth fp32-oracle check of the workload")
     ap.add_argument("--no-ep", action="store_true", help="N > 1: skip the expert-parallel configs[3] record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results (rank 0) to DIR/<name>.npy: generated_ids, "
+                         "prefill_hidden (the prefill's last-layer hidden states), decode_hidden (the last decode "
+                         "step's last-layer hidden state)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -189,3 +189,17 @@ def sample_frame_positions(n_frames: int, fps: float, max_frames: int, min_frame
     if len(all_pos) < min_frames:
         return [all_pos[i] for i in np.linspace(0, len(all_pos) - 1, num=min_frames, dtype=int)]
     return all_pos
+
+
+# ------------------------------------------------------------------------------------------------ golden inputs
+def card(h: int, w: int, k: int) -> np.ndarray:
+    """Deterministic integer test card: gradients, a checkerboard patch, hard-edged boxes (no libm, no RNG).  The image
+    golden stores (h, w, k) and a digest of each card rather than its pixels."""
+    yy, xx = np.mgrid[0:h, 0:w].astype(np.int64)
+    img = np.stack([(xx * 255 // max(w - 1, 1) + k * 17) % 256, (yy * 255 // max(h - 1, 1) + k * 29) % 256,
+                    ((xx + yy) * 3 + k * 41) % 256], -1)
+    cb = ((xx // 7 + yy // 5) % 2 == 0) & (xx > w // 2) & (yy < h // 2)
+    img[cb] = 255 - img[cb]
+    img[h // 3: h // 3 + max(h // 9, 2), w // 4: w // 4 + max(w // 5, 2)] = (250, 10, 128)
+    img[(yy - h // 2) ** 2 + (xx - w // 3) ** 2 < (min(h, w) // 6) ** 2] = (5, 240, 60)
+    return img.astype(np.uint8)

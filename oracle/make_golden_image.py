@@ -3,17 +3,22 @@
     functions are compiled from the reference source without importing the training module) driving Pillow's resize;
   * pixel values: transformers' CLIPImageProcessor with the reference's preprocessor_config.json constants, cast to
     bf16 as `model.process_images(...).to(dtype=model.dtype)` does (video_audio_demo.py:219-221).
-Inputs are stored; outputs are stored as SHA-256 digests plus a small crop (the numpy oracle reproduces them bit for
-bit, tests/test_image.py).  Run: python oracle/make_golden_image.py"""
+Inputs are oracle.image_oracle.card test cards, stored as their (h, w, k) and a SHA-256 digest; outputs are stored as
+SHA-256 digests plus a small crop (the numpy oracle reproduces them bit for bit, tests/test_image.py).
+Run: python oracle/make_golden_image.py"""
 import ast
 import hashlib
 import os
+import sys
 
 import numpy as np
 import torch
 from PIL import Image
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE))
+from oracle.image_oracle import card  # noqa: E402
+
 REF = "/root/reference/vita/util/data_utils_video_audio_neg_patch.py"
 
 
@@ -23,18 +28,6 @@ def reference_functions():
         if isinstance(node, ast.FunctionDef) and node.name in ("find_closest_aspect_ratio", "dynamic_preprocess"):
             exec(compile(ast.Module([node], []), REF, "exec"), ns)
     return ns["dynamic_preprocess"]
-
-
-def pattern(h: int, w: int, k: int) -> np.ndarray:
-    """Deterministic integer test card: gradients, a checkerboard patch, hard-edged boxes (no libm, no RNG)."""
-    yy, xx = np.mgrid[0:h, 0:w].astype(np.int64)
-    img = np.stack([(xx * 255 // max(w - 1, 1) + k * 17) % 256, (yy * 255 // max(h - 1, 1) + k * 29) % 256,
-                    ((xx + yy) * 3 + k * 41) % 256], -1)
-    cb = ((xx // 7 + yy // 5) % 2 == 0) & (xx > w // 2) & (yy < h // 2)
-    img[cb] = 255 - img[cb]
-    img[h // 3: h // 3 + max(h // 9, 2), w // 4: w // 4 + max(w // 5, 2)] = (250, 10, 128)
-    img[(yy - h // 2) ** 2 + (xx - w // 3) ** 2 < (min(h, w) // 6) ** 2] = (5, 240, 60)
-    return img.astype(np.uint8)
 
 
 def sha(a) -> str:
@@ -49,11 +42,12 @@ def main():
     out = {}
     cases = {"wide": (300, 500, 1), "tall": (451, 167, 2), "square": (448, 448, 3), "tiny": (37, 61, 4), "pano": (120, 950, 5)}
     for name, (h, w, k) in cases.items():
-        img = pattern(h, w, k)
+        img = card(h, w, k)
         tiles, n = dyn(Image.fromarray(img), min_num=1, max_num=12, image_size=448, use_thumbnail=True)
         t = np.stack([np.asarray(x) for x in tiles])
         pv = ip.preprocess(list(tiles), return_tensors="pt")["pixel_values"].to(torch.bfloat16)
-        out[name + "_image"] = img
+        out[name + "_image_card"] = np.array([h, w, k])
+        out[name + "_image_sha256"] = np.array(sha(img))
         out[name + "_tiles_sha256"] = np.array(sha(t))
         out[name + "_pixels_bf16_sha256"] = np.array(sha(pv.view(torch.int16).numpy()))
         out[name + "_n_tiles"] = np.array(n[0])
@@ -78,8 +72,9 @@ def main():
     frames = {"landscape": (180, 320, 6), "portrait": (321, 179, 7), "sq": (200, 200, 8)}
     bg = tuple(int(x * 255) for x in ipp.image_mean)
     for name, (h, w, k) in frames.items():
-        img = pattern(h, w, k)
-        out["frame_" + name] = img
+        img = card(h, w, k)
+        out["frame_" + name + "_card"] = np.array([h, w, k])
+        out["frame_" + name + "_sha256"] = np.array(sha(img))
         for pad in (True, False):
             pil = Image.fromarray(img)
             pv = ipp.preprocess(expand2square(pil, bg) if pad else pil, return_tensors="pt")["pixel_values"].to(torch.bfloat16)

@@ -3,15 +3,15 @@ CLIP normalisation (oracle/image_oracle.py) against the golden digests minted fr
 `dynamic_preprocess`, Pillow and transformers (oracle/make_golden_image.py) -- bit for bit -- and the host-side
 coefficient tables / lookup table of vita_b200.image_frontend against the oracle's."""
 import hashlib
-import os
 
 import numpy as np
 import pytest
 import torch
 
 from oracle import image_oracle as O
+from tests.util import load_image_golden
 
-GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "image_golden.npz"))
+GOLD = load_image_golden()
 CASES = ["wide", "tall", "square", "tiny", "pano"]
 
 

@@ -2,16 +2,16 @@
 CLIPImageProcessor, minted by oracle/make_golden_image.py) and against the numpy oracle: integer / byte work, so the bar
 is bit-exact."""
 import hashlib
-import os
 
 import numpy as np
 import pytest
 import torch
 
 from oracle import image_oracle as O
+from tests.util import load_image_golden
 
 pytestmark = pytest.mark.gpu
-GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "image_golden.npz"))
+GOLD = load_image_golden()
 
 
 def sha(a) -> str:

@@ -1,7 +1,23 @@
 """Shared helpers for the parity tests (the oracle is imported here as the checker only)."""
+import hashlib
+from pathlib import Path
+
+import numpy as np
 import torch
 
 BF16 = torch.bfloat16
+
+
+def load_image_golden() -> dict:
+    """tests/golden/image_golden.npz with every input image rebuilt from its stored (h, w, k) test-card recipe
+    (`<key>_card`) and checked against the digest of the card the outputs were minted from (`<key>_sha256`)."""
+    from oracle.image_oracle import card
+    g = dict(np.load(Path(__file__).resolve().parent / "golden" / "image_golden.npz"))
+    for key in [k[: -len("_card")] for k in g if k.endswith("_card")]:
+        img = card(*g.pop(key + "_card").tolist())
+        assert hashlib.sha256(img.tobytes()).hexdigest() == str(g.pop(key + "_sha256")), f"{key}: test card differs"
+        g[key] = img
+    return g
 
 
 def bf16_round(t: torch.Tensor) -> torch.Tensor:
